@@ -218,6 +218,24 @@ def reference_arm(a, rank):
     emit(line)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, cs, ctx):
+    """Writes the result of the last cull as its caller receives it: the visible ids grouped by renderable type (sorted inside a type,
+    where their order is unspecified) and the per-type counts, as float64 .npy files.  A list over the size limit is written as a
+    fixed, seeded sample of its entries."""
+    ptr, res = cs.last_result()
+    counts = np.array(res.type_count[:res.n_types], np.int64)
+    ids = [np.sort(ctx.copy_to_host(ptr + 4 * int(res.type_offset[t]), int(c), np.uint32)) for t, c in enumerate(counts) if c]
+    ids = np.concatenate(ids).astype(np.float64) if ids else np.zeros(0)
+    if ids.nbytes + counts.nbytes > DUMP_BYTES:
+        ids = ids[np.sort(np.random.default_rng(0).choice(len(ids), (DUMP_BYTES - counts.nbytes) // 8, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "visible_ids.npy"), ids)
+    np.save(os.path.join(out_dir, "visible_type_counts.npy"), counts.astype(np.float64))
+
+
 def time_region(ctx, fn, steps):
     e0, e1 = ctx.event(), ctx.event()
     ctx.synchronize()
@@ -575,6 +593,8 @@ def ours(a, rank, world):
         ms_total = float(t.item())
         dist.barrier()
     ms_step = ms_total / a.steps
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, cs, ctx)
 
     # N>1, bitmask exchange: one exchanged step is checked — what every rank sees of rank r's slab (per-type counts, visibility rows by page
     # id) must be what rank r holds itself, and rank r's own rows must say exactly what its own cull made visible
@@ -782,7 +802,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--only-cull", action="store_true", help="skip the secondary paths and the CPU baseline leg (profiling runs)")
     ap.add_argument("--no-c5", action="store_true", help="skip the 50M + 1M mixed scene (BASELINE configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the visible set of the last timed cull (rank 0's shard at N>1) to DIR/*.npy, "
+                                                          "so that two builds can be compared output for output: the inputs are seeded")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3)
     claim_stdout()
     rank = int(os.environ.get("RANK", "0"))

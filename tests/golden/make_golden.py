@@ -96,8 +96,11 @@ def math_kat():
     r = np.zeros(64, np.float32)
     L.ref_rng_floats(C.c_uint32(521288629), C.c_uint32(362436069), C.c_uint32(64), P(r), None)
     d.update(rng64=r)
-    np.savez_compressed(os.path.join(OUT, "math_kat.npz"), **d)
-    print("math_kat.npz", sum(v.nbytes for v in d.values()))
+    # two files, each under 1 MB: the cell / frustum / RNG vectors go to math_kat_frustum.npz
+    frustum = ("cell_pos", "cell_idx", "fr_args", "fr_out", "rel_origin", "rel_out", "box_pos", "box_size", "box_contains", "box_intersects", "rng64")
+    np.savez_compressed(os.path.join(OUT, "math_kat.npz"), **{k: v for k, v in d.items() if k not in frustum})
+    np.savez_compressed(os.path.join(OUT, "math_kat_frustum.npz"), **{k: d[k] for k in frustum})
+    print("math_kat.npz + math_kat_frustum.npz", sum(v.nbytes for v in d.values()))
 
 
 def cull_kat():
@@ -329,15 +332,146 @@ def sortkeys_kat():
     print("sortkeys_kat.npz", sum(v.nbytes for v in d.values()))
 
 
+def digest(*arrays):
+    """16-byte digest of the bytes of `arrays` (tests/test_oracle_ref.py computes the same over the restatement's outputs)."""
+    import hashlib
+    h = hashlib.blake2b(digest_size=16)
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return np.frombuffer(h.digest(), np.uint8)
+
+
+def record_cull(d, key, ids, tys, info):
+    """A visible set of the reference's cull: count, result pages and the digest of the ids in ascending order with their types."""
+    o = np.argsort(ids)
+    d[f"{key}_info"], d[f"{key}_digest"] = np.array([info["count"], info["pages"]], np.int64), digest(ids[o].astype(np.uint32), tys[o].astype(np.uint8))
+
+
+def cull_sets(workers, out):
+    """The scene and views of test_cull_sets_equal_reference_job_system through the reference's cull on a job system of `workers` workers.
+    The job system is process-wide, so every worker count is recorded by a process of its own."""
+    scene = scenes.cull_scene(400_000, (3000.0, 300.0, 3000.0), seed=123, big_fraction=0.005, type_probs=(0.5, 0.3, 0.2))
+    rc = po.RefCulling(workers=workers)
+    assert rc.workers == workers
+    rc.add(scene["entities"], scene["types"], scene["pos"], scene["radius"])
+    d = {}
+    for v, a in enumerate((scenes.c1_frustum_args(), dict(scenes.c1_frustum_args(), position=(900.0, -50.0, 400.0), direction=(-0.7, 0.1, -0.7), far=3500.0))):
+        fr = po.ref_frustum_perspective(a["position"], a["direction"], a["up"], a["fov"], a["ratio"], a["near"], a["far"])
+        ids, tys, info = rc.cull(fr, cap=len(scene["entities"]), iters=2)
+        d[f"sets_w{workers}_v{v}_frustum"] = fr
+        record_cull(d, f"sets_w{workers}_v{v}", ids, tys, info)
+    np.savez(out, **d)
+
+
+def ref_crosscheck():
+    """What the reference's own code returned in the cross-checks of tests/test_oracle_ref.py and tests/test_sortkeys_oracle.py: the same
+    seeded inputs, in the same order, through the reference build instead of the restatement."""
+    import subprocess
+    import tempfile
+    L = po.ref()
+    names = ["Sphere", "Frustum", "ShiftedFrustum", "ShiftedFrustum.origin", "Transform", "CullResult", "CullResult.entities", "LocalRigidTransform", "DualQuat", "Matrix"]
+    d = dict(sizeof_names=np.array(names), sizeof_values=np.array([L.ref_sizeof(k.encode()) for k in names], np.int64))
+    with tempfile.TemporaryDirectory() as tmp:
+        for w in (1, 4):
+            subprocess.check_call([sys.executable, os.path.abspath(__file__), "--cull-sets", str(w), os.path.join(tmp, f"w{w}.npz")])
+            d.update(np.load(os.path.join(tmp, f"w{w}.npz")))
+    # random worlds, views and edits (test_random_views_and_edits_equal_reference)
+    rng = np.random.default_rng(2024)
+    for world in range(3):
+        n = int(rng.integers(2_000, 30_000))
+        half = (float(rng.choice([250.0, 900.0, 4000.0])), float(rng.choice([50.0, 400.0])), float(rng.choice([250.0, 900.0, 4000.0])))
+        scene = scenes.cull_scene(n, half, seed=300 + world, big_fraction=float(rng.choice([0.0, 0.02, 0.3])), type_probs=(0.5, 0.25, 0.25))
+        rc = po.RefCulling(workers=1)
+        rc.add(scene["entities"], scene["types"], scene["pos"], scene["radius"])
+        alive = np.ones(n, bool)
+        pos, rad = scene["pos"].copy(), scene["radius"].copy()
+        for step in range(12):
+            p = rng.normal(size=3) * np.array(half) * 1.5
+            dv = rng.normal(size=3); dv /= np.linalg.norm(dv)
+            up = np.cross(np.cross(dv, rng.normal(size=3)), dv); up /= np.linalg.norm(up)
+            if step % 5 == 0:
+                p = np.round(p / 300.0) * 300.0
+                dv, up = np.array([0.0, 0.0, -1.0]), np.array([0.0, 1.0, 0.0])
+            far = float(rng.choice([30.0, 700.0, 5000.0, 60000.0]))
+            if step % 3 == 2:
+                args = (p, dv.astype(np.float32), up.astype(np.float32), float(rng.uniform(10, 3000)), float(rng.uniform(10, 3000)), 0.0, far)
+                fr = po.ref_frustum_ortho(*args)
+            else:
+                args = (p, dv.astype(np.float32), up.astype(np.float32), float(rng.uniform(0.2, 2.4)), float(rng.uniform(0.5, 2.5)), float(rng.uniform(0.01, 2.0)), far)
+                fr = po.ref_frustum_perspective(*args)
+            t = int(rng.choice([-1, -1, 0, 1, 2]))
+            ids, tys, info = rc.cull(fr, type=t, cap=n, iters=1)
+            d[f"rv{world}_{step}_frustum"] = fr
+            record_cull(d, f"rv{world}_{step}", ids, tys, info)
+            live = np.nonzero(alive)[0]
+            mv = rng.choice(live, min(len(live), 400), replace=False).astype(np.int32)
+            a, b, c = np.array_split(mv, 3)
+            pos[a] = pos[a] + rng.normal(size=(len(a), 3)) * 200.0
+            rc.set_position(a, pos[a])
+            rad[b] = (rng.random(len(b)) * 500.0).astype(np.float32)
+            rc.set_radius(b, rad[b])
+            rc.remove(c)
+            alive[c] = False
+    # random clips (test_random_clips_equal_reference): digests of the reference's poses (positions, then rotations) in the order the test asks for them
+    rng = np.random.default_rng(99)
+    digests = []
+    for trial in range(25):
+        bones = int(rng.choice([1, 2, 3, 4, 5, 7, 16, 33, 64, 100, 196]))
+        frames = int(rng.integers(1, 91))
+        pb = tuple(int(x) for x in rng.integers(3, 20, 3))
+        rb = tuple(int(x) for x in rng.integers(3, 20, 3))
+        sk = scenes.skeleton(bones, seed=500 + trial)
+        clip = scenes.clip(sk, frames=frames, fps=float(rng.choice([1.0, 24.0, 30.0, 59.94])), seed=600 + trial, pos_bits=pb, rot_bits=rb,
+                           const_fraction=float(rng.choice([0.0, 0.25, 1.0])))
+        other = scenes.clip(sk, frames=int(rng.integers(1, 40)), seed=700 + trial, const_fraction=0.5)
+        Lt = clip.length_ticks
+        for t in [0, 1, max(Lt - 1, 0), Lt, Lt + 5000] + [int(x) for x in rng.integers(0, max(Lt, 1), 6)]:
+            for absolute in (False, True):
+                digests.append(digest(*po.ref_pose_evaluate(sk, clip, t, compute_absolute=absolute)))
+            rel = po.ref_pose_evaluate(sk, clip, t, compute_absolute=False)
+            w = float(rng.choice([0.0, 0.3, 0.9998, 0.9999, 1.0]))
+            t2 = int(rng.integers(0, max(other.length_ticks, 1)))
+            digests.append(digest(*po.ref_pose_evaluate(sk, other, t2, weight=w, start_from_bind=False, compute_absolute=True, pos=rel[0], rot=rel[1])))
+    d["clip_digests"] = np.array(digests)
+    # exact thresholds (test_threshold_values_equal_reference): the restatement's frusta, the reference's cull
+    r_edge = np.float32(300.0)
+    radii = np.array([r_edge, np.nextafter(r_edge, np.float32(1e9)), np.nextafter(r_edge, np.float32(0)), 0.0, 1e-30], np.float32)
+    coords = [0.0, -0.0, 300.0, -300.0, 299.99999999, -299.99999999, 300.00000001, 600.0, -600.0, 899.9999, 1e-300, -1e-300]
+    pos = np.array([[x, y, 10.0] for x in coords for y in (0.0, -300.0, 299.99999999)], np.float64)
+    n = len(pos) * len(radii)
+    P_, R = np.repeat(pos, len(radii), axis=0), np.tile(radii, len(pos))
+    E = np.arange(n, dtype=np.int32)
+    rc = po.RefCulling(workers=1)
+    rc.add(E, (E % 3).astype(np.uint8), P_, R)
+    a = scenes.c1_frustum_args()
+    for v, args in enumerate((dict(a, position=(0.0, 0.0, 500.0)), dict(a, position=(300.0, 0.0, 300.0), direction=(-1.0, 0.0, 0.0)),
+                              dict(a, position=(-1000.0, 100.0, 0.0), direction=(1.0, 0.0, 0.0), far=5000.0))):
+        f = po.frustum_perspective(args["position"], args["direction"], args["up"], args["fov"], args["ratio"], args["near"], args["far"])
+        record_cull(d, f"th_v{v}", *rc.cull(f, cap=n, iters=1))
+    big, edge = E[R > r_edge], E[R == r_edge]
+    rc.set_radius(big, np.full(len(big), r_edge, np.float32))
+    rc.set_radius(edge, np.full(len(edge), np.nextafter(r_edge, np.float32(1e9)), np.float32))
+    f = po.frustum_perspective(a["position"], a["direction"], a["up"], a["fov"], a["ratio"], a["near"], 5000.0)
+    record_cull(d, "th_edited", *rc.cull(f, cap=n, iters=1))
+    # PipelineImpl::radixSort on its job system (test_reference_build_agrees_live)
+    rng = np.random.default_rng(5)
+    for size in (0, 1, 300, 700, 4096):
+        keys = (rng.integers(0, 4, size).astype(np.uint64) << np.uint64(56)) | rng.integers(0, 1 << 20, size).astype(np.uint64)
+        d[f"rs{size}_digest"] = digest(*po.ref_radix_sort(keys, np.arange(size, dtype=np.uint64), workers=2))
+    np.savez_compressed(os.path.join(OUT, "ref_crosscheck.npz"), **d)
+    print("ref_crosscheck.npz", sum(v.nbytes for v in d.values()))
+
+
 if __name__ == "__main__":
     po.build()
+    if sys.argv[1:2] == ["--cull-sets"]:
+        cull_sets(int(sys.argv[2]), sys.argv[3])
+        sys.stdout.flush()
+        os._exit(0)
     po.ref().ref_clip_length_ticks.restype = C.c_uint32
     po.ref().ref_time_from_seconds.restype = C.c_uint32
-    math_kat()
-    pose_kat()
-    cull_kat()
-    world_kat()
-    ani_kat()
-    sortkeys_kat()
+    # python tests/golden/make_golden.py [name ...]: only the named sets (default: all)
+    for name in sys.argv[1:] or ["math_kat", "pose_kat", "cull_kat", "world_kat", "ani_kat", "sortkeys_kat", "ref_crosscheck"]:
+        globals()[name]()
     sys.stdout.flush()
     os._exit(0)

@@ -1,4 +1,4 @@
-"""Multi-GPU path on real devices (needs >= 2 GPUs: `gpurun --gpus 2`): each rank culls its index-range shard on its own GPU,
+"""Multi-GPU path on real devices (needs >= 2 GPUs): each rank culls its index-range shard on its own GPU,
 lb200_culling_allgather exchanges the compacted visible lists over NCCL, and the merged result equals the oracle's unsharded cull.
 The bitmask exchange fused into the cull kernel (lb200_culling_cull_exchange) is also run with a world of ONE rank, so that its
 peer-store / epoch-flag path is covered on a single-GPU box."""
@@ -193,14 +193,14 @@ def test_bitmask_exchange_one_rank():
 def test_bitmask_exchange_two_gpus():
     import lumixengine_b200 as lb
     if lb.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     _run(_exchange_worker, 2)
 
 
 def test_two_gpu_cull_allgather():
     import lumixengine_b200 as lb
     if lb.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import torch.multiprocessing as mp
     mpctx = mp.get_context("spawn")
     q = mpctx.Queue()

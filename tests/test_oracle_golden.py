@@ -19,7 +19,7 @@ def bits(a):
 
 @pytest.fixture(scope="module")
 def kat():
-    return np.load(os.path.join(G, "math_kat.npz"))
+    return {**np.load(os.path.join(G, "math_kat.npz")), **np.load(os.path.join(G, "math_kat_frustum.npz"))}
 
 
 def test_math_primitives_bit_exact(oracle, kat):

@@ -1,11 +1,11 @@
 """CPU: the sort-key oracle (oracle/oracle_sortkeys.c) against vectors the reference's own code produced (tests/golden/sortkeys_kat.npz:
-packers, Model::getLODMeshIndices and PipelineImpl::radixSort cut out of pipeline.cpp / model.h by oracle/build_ref.sh), live against
-that build where it exists, and properties of the createSortKeys restatement."""
+packers, Model::getLODMeshIndices and PipelineImpl::radixSort cut out of pipeline.cpp / model.h by oracle/build_ref.sh, and
+tests/golden/ref_crosscheck.npz: its radix sort on its job system), and properties of the createSortKeys restatement."""
 import ctypes as C
+import hashlib
 import os
 
 import numpy as np
-import pytest
 
 from lumixengine_b200 import scenes, sortkeys
 
@@ -42,20 +42,15 @@ def test_radix_sort_matches_reference_vectors(oracle):
 
 
 def test_reference_build_agrees_live(oracle):
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built here")
-    try:
-        R = oracle.sortkey_packers("ref")
-    except AttributeError:
-        pytest.skip("oracle/_ref was built without the sort-key harness")
-    _packers_equal(R, G)
+    """PipelineImpl::radixSort of the reference build on its job system against the restatement: the digest of the sorted keys and values
+    (tests/golden/ref_crosscheck.npz)."""
+    R = np.load(os.path.join(os.path.dirname(__file__), "golden", "ref_crosscheck.npz"))
     rng = np.random.default_rng(5)
     for size in (0, 1, 300, 700, 4096):
         keys = (rng.integers(0, 4, size).astype(np.uint64) << np.uint64(56)) | rng.integers(0, 1 << 20, size).astype(np.uint64)
         vals = np.arange(size, dtype=np.uint64)
-        rk, rv = oracle.ref_radix_sort(keys, vals, workers=2)
         ok, ov = oracle.radix_sort(keys, vals, reference_copy_back=True)
-        assert np.array_equal(rk, ok) and np.array_equal(rv, ov), size
+        assert hashlib.blake2b(ok.tobytes() + ov.tobytes(), digest_size=16).digest() == R[f"rs{size}_digest"].tobytes(), size
 
 
 def _inputs(n=20000, seed=3):
